@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """480p frames/sec of the exemplar-colorization forward path on N B200s + correlation-kernel roofline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): one 480x854 grayscale frame + 1 exemplar, replicate-padded to the
 legal 480x864 (SURVEY.md fact 2: the reference rejects W % 16 != 0), N = 120*216 = 25920 positions.
@@ -23,6 +23,10 @@ Timed legs (own arm):
   cpu_baseline : the CPU oracle (port of the reference's PyTorch forward) on the host cores, bounded sample.
 Reference arm (--impl reference): the same CPU oracle timed step by step on rank 0 (the reference is pure
 Python/PyTorch and cannot travel to the GPU box; oracle/dvc_oracle.py is bit-exact with it, tests/golden/PIN_REPORT.txt).
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the timed path returned for its last step, DIR/ab.npy
+(float32 [1,2,480,864], 3.3 MB).  Inputs and weights are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import json
@@ -157,8 +161,18 @@ def pick_cpu_threads(sds):
     return best
 
 
+def dump_outputs(out_dir, **arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy in float32."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().to(torch.float32).cpu().numpy())
+
+
 def cpu_frames_per_sec(n_timed, warm=1):
-    """The CPU oracle (= the reference's PyTorch CPU forward, bit-exact port) on this host's cores."""
+    """The CPU oracle (= the reference's PyTorch CPU forward, bit-exact port) on this host's cores.
+    Returns the step times, the thread count and the ab of the last step."""
     from dvc.synth import make_state_dict
     from oracle import dvc_oracle as O
 
@@ -178,7 +192,7 @@ def cpu_frames_per_sec(n_timed, warm=1):
             if t >= warm:
                 times.append(dt)
             last = torch.cat((frames[t:t + 1], ab), 1)
-    return times, cores
+    return times, cores, ab
 
 
 def run_reference(args, rank):
@@ -186,7 +200,9 @@ def run_reference(args, rank):
     if rank != 0:
         return
     t_all = time.perf_counter()
-    times, cores = cpu_frames_per_sec(args.steps, warm=max(args.warmup, 1))
+    times, cores, ab = cpu_frames_per_sec(args.steps, warm=max(args.warmup, 1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ab=ab)
     total = sum(times)
     fps = len(times) / total
     line = {
@@ -235,7 +251,11 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=4, help="frames timed for cpu_baseline (0 = skip)")
     ap.add_argument("--sustain-s", type=float, default=2.5, help="length of the extra sustained run of the headline (0 = skip)")
     ap.add_argument("--clip-frames", type=int, default=64, help="frames of the config-3 clip (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "own" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -425,6 +445,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ab=dev_out[K - 1:K])  # the value leg's last frame; no later leg writes dev_out
 
     peak, peak_src = measured_peak(ms_serial * KP * 1e-3)
     achieved = CORR_FLOP / (corr_ms * 1e-3) / 1e12 if corr_ms > 0 else 0.0
@@ -488,7 +510,7 @@ def main():
     }
     if args.cpu_sample > 0:
         tb = time.perf_counter()
-        times, cores = cpu_frames_per_sec(args.cpu_sample, warm=1)
+        times, cores, _ = cpu_frames_per_sec(args.cpu_sample, warm=1)
         line["cpu_baseline"] = {"value": len(times) / sum(times), "unit": "frames/s", "cores": cores, "kind": "port",
                                 "sample": f"{len(times)} frames of the same workload after 1 warm-up frame "
                                           f"({time.perf_counter() - tb:.0f} s of CPU work)"}

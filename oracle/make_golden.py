@@ -21,6 +21,7 @@ Cases (all legal shapes: H % 8 == 0, W % 16 == 0):
   cfg1_256x256     B=1, T=1e-10            BASELINE.json configs[0]; outputs only, inputs regenerated from the seed
   default_480x864  B=1, T=1e-10            BASELINE.json configs[1], the bench size (N = 25920); outputs only, inputs
                                            regenerated from the seed (make_lab(seed), make_lab(seed+1), make_lab(seed+2)*0.5)
+  contextual_loss  ContextualLoss_forward  models/ContextualLoss.py on the seeded maps of contextual_loss_maps(); outputs only
 
     python oracle/make_golden.py --only default_480x864     # (re)generate one case, keep the others untouched
 """
@@ -148,6 +149,29 @@ def run_clip(ns, name, F_, H, W, seed):
     return {"oracle32_vs_ref32_ab": float((mine - ref).abs().max())}
 
 
+def contextual_loss_maps():
+    """(key, X, Y, feature_centering) of the contextual-loss case: seeded ReLU feature maps of several depths."""
+    g = torch.Generator().manual_seed(31)
+    for (B, C, h, w) in ((2, 128, 12, 16), (1, 256, 16, 16), (1, 512, 8, 12)):
+        X = torch.relu(torch.randn(B, C, h, w, generator=g))
+        Y = torch.relu(torch.randn(B, C, h, w, generator=g) + 0.3 * X)
+        for centering in (True, False):
+            yield f"loss_{C}_{int(centering)}", X, Y, centering
+
+
+def run_contextual_loss(ns, name):
+    torch.set_num_threads(8)
+    mod = ns.ContextualLoss_forward()
+    out, report = {}, {}
+    with torch.no_grad():
+        for key, X, Y, centering in contextual_loss_maps():
+            ref = mod(X.clone(), Y.clone(), 0.1, centering)
+            report[f"oracle32_vs_ref32_{key}"] = float((O.contextual_loss_forward(X, Y, 0.1, centering) - ref).abs().max())
+            out[key] = npf(ref)
+    np.savez_compressed(os.path.join(GOLD, name + ".npz"), **out)
+    return report
+
+
 def write_report(lines, replace_all):
     """PIN_REPORT.txt: one section per case; --only replaces just that case's section."""
     path = os.path.join(GOLD, "PIN_REPORT.txt")
@@ -208,6 +232,10 @@ def main():
         rep = run_clip(ns, "clip3_32x48", 3, 32, 48, 707)
         print("[clip3_32x48]", rep)
         lines.append(("clip3_32x48", rep))
+    if not args.only or args.only == "contextual_loss":
+        rep = run_contextual_loss(ns, "contextual_loss")
+        print("[contextual_loss]", rep)
+        lines.append(("contextual_loss", rep))
     write_report(lines, replace_all=not args.only)
 
 

@@ -1,9 +1,8 @@
-"""Import the UNMODIFIED reference modules from /root/reference (build container only).
+"""Import the UNMODIFIED reference modules from a checkout of the reference (REF_ROOT below).
 
-TEST INFRASTRUCTURE.  /root/reference does not exist on the GPU box, so nothing under
-`-m gpu`, smoke() or bench.py may call this; it is used by oracle/make_golden.py (fixture
-generation) and by the CPU-only test that pins oracle/dvc_oracle.py to the reference when the
-tree is present.
+FIXTURE GENERATION ONLY.  The reference is not part of this repository, so no test, smoke() or
+bench.py may call this; oracle/make_golden.py uses it to write tests/golden/, which the tests
+compare against.
 
 Three shims are needed (SURVEY.md §8c):
   1. utils/util.py:6,10 import matplotlib.pyplot and skimage at module top (absent here);

@@ -151,30 +151,32 @@ def test_exemplar_broadcast_world2_gloo(tmp_path):
         assert p.returncode == 0 and "OK" in o, o
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference tree not present (GPU box)")
-def test_dropin_import_resolution_with_reference_tree():
+def test_dropin_import_resolution_with_reference_tree(tmp_path):
     """INTEGRATION.md §1: with the package ahead of the reference on sys.path, `models.NonlocalNet` /
-    `models.ColorVidNet` are the drop-ins while `models.FrameColor` is still the reference's own file."""
+    `models.ColorVidNet` are the drop-ins while `models.FrameColor` is still the reference's own file.  The reference tree
+    is stood in for by its layout: `models/` without __init__.py, holding its own NonlocalNet / ColorVidNet (which fail if
+    they are ever imported) and FrameColor."""
+    ref = tmp_path / "reference"
+    (ref / "models").mkdir(parents=True)
+    for mod in ("NonlocalNet", "ColorVidNet"):
+        (ref / "models" / f"{mod}.py").write_text(f"raise ImportError('the reference {mod} shadowed the drop-in')\n")
+    (ref / "models" / "FrameColor.py").write_text("def frame_colorization(*args, **kwargs):\n    raise NotImplementedError\n")
     code = r"""
-import sys, types
-for n in ["matplotlib", "matplotlib.pyplot", "skimage", "skimage.color", "skimage.io"]:
-    sys.modules.setdefault(n, types.ModuleType(n))
-sys.modules["matplotlib"].pyplot = sys.modules["matplotlib.pyplot"]
-sys.modules["skimage"].color = sys.modules["skimage.color"]; sys.modules["skimage"].io = sys.modules["skimage.io"]
-sys.path.insert(0, "/root/reference"); sys.path.insert(0, sys.argv[1])
+import os, sys
+sys.path.insert(0, sys.argv[2]); sys.path.insert(0, sys.argv[1])
 import models
-models.__path__.append("/root/reference/models")
+models.__path__.append(os.path.join(sys.argv[2], "models"))
 from models.NonlocalNet import VGG19_pytorch, WarpNet
 from models.ColorVidNet import ColorVidNet
 from models.FrameColor import frame_colorization
 import models.NonlocalNet as N, models.FrameColor as F
 assert sys.argv[1] in N.__file__, N.__file__
-assert F.__file__.startswith("/root/reference/"), F.__file__
+assert F.__file__.startswith(sys.argv[2]), F.__file__
 assert "dvc" in N.__dict__            # the drop-in imports the ctypes binding, the reference's file does not
 print("RESOLVED")
 """
     pkg = os.path.join(ROOT, "deep-exemplar-based-video-colorization_b200")
-    out = subprocess.run([sys.executable, "-c", code, pkg], capture_output=True, text=True, timeout=120)
+    out = subprocess.run([sys.executable, "-c", code, pkg, str(ref)], capture_output=True, text=True, timeout=120)
     assert out.returncode == 0 and "RESOLVED" in out.stdout, out.stdout + out.stderr
 
 
