@@ -10,6 +10,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <map>
 #include <string>
 #include <unordered_map>
@@ -163,6 +164,13 @@ struct dvc_ctx {
   cudaEvent_t evA[4] = {nullptr, nullptr, nullptr, nullptr}, evC[4] = {nullptr, nullptr, nullptr, nullptr}, evFork = nullptr,
               evJoinA = nullptr, evJoinC = nullptr, evJoinD = nullptr;
   cudaEvent_t evU[4] = {nullptr, nullptr, nullptr, nullptr}, evD[4] = {nullptr, nullptr, nullptr, nullptr};
+  // video driver (dvc_colorize_video_rgb8): post-processing + download stream, one event per batch slot of the rings
+  cudaStream_t sP = nullptr;
+  cudaEvent_t evP[2] = {nullptr, nullptr}, evJoinP = nullptr;
+  int video_batch = 8;  // frames per dvc_postprocess_rgb8 batch in the video driver (DESIGN.md §4.5: measured)
+  // recurrence state of dvc_colorize_video_rgb8 ("vid.last"): valid for this exemplar version and output size only
+  long long vid_ex_version = -1;
+  int vid_Ho = 0, vid_Wo = 0;
   // exemplar cache
   float* ex_phi = nullptr;  // [N][256]
   float* ex_V = nullptr;    // [N][4]
@@ -1115,6 +1123,10 @@ extern "C" int dvc_destroy(dvc_ctx* c) {
   if (c->evJoinD) cudaEventDestroy(c->evJoinD);
   if (c->sU) cudaStreamDestroy(c->sU);
   if (c->sD) cudaStreamDestroy(c->sD);
+  if (c->sP) cudaStreamDestroy(c->sP);
+  for (int i = 0; i < 2; ++i)
+    if (c->evP[i]) cudaEventDestroy(c->evP[i]);
+  if (c->evJoinP) cudaEventDestroy(c->evJoinP);
   if (c->ex_phi) cudaFree(c->ex_phi);
   if (c->ex_V) cudaFree(c->ex_V);
   corr_ws_free(&c->corr_ws);
@@ -1148,6 +1160,7 @@ extern "C" int dvc_debug_set_flag(dvc_ctx* c, const char* name, int value) {
     return DVC_OK;
   }
   if (!strcmp(name, "clip_astreams")) { c->clip_astreams = value == 2 ? 2 : 1; return DVC_OK; }
+  if (!strcmp(name, "video_batch")) { c->video_batch = value < 1 ? 1 : (value > 64 ? 64 : value); return DVC_OK; }  // measurements
   if (!strcmp(name, "tc_tail")) { c->tc_tail = value < 0 ? 0 : value; return DVC_OK; }  // > 1: pretend pair-slot count (tests)
   if (!strcmp(name, "tc_f16")) { c->tc_f16 = value != 0; return DVC_OK; }
   if (!strcmp(name, "tc_splits")) { c->tc_splits = value < 0 ? 0 : (value > 8 ? 8 : value); return DVC_OK; }
@@ -1651,56 +1664,52 @@ static int clip_streams(dvc_ctx* c) {
   CUDA_TRY(c, cudaEventCreateWithFlags(&c->evFork, cudaEventDisableTiming));
   CUDA_TRY(c, cudaEventCreateWithFlags(&c->evJoinA, cudaEventDisableTiming));
   CUDA_TRY(c, cudaEventCreateWithFlags(&c->evJoinC, cudaEventDisableTiming));
+  CUDA_TRY(c, cudaStreamCreateWithFlags(&c->sP, cudaStreamNonBlocking));
+  CUDA_TRY(c, cudaEventCreateWithFlags(&c->evP[0], cudaEventDisableTiming));
+  CUDA_TRY(c, cudaEventCreateWithFlags(&c->evP[1], cudaEventDisableTiming));
+  CUDA_TRY(c, cudaEventCreateWithFlags(&c->evJoinP, cudaEventDisableTiming));
   return DVC_OK;
 }
 
-// test.py:68-96 for one contiguous segment.  Frame t+1's frame-independent phase (VGG / WarpNet / correlation)
-// runs on stream A while frame t's ColorVidNet -- which needs frame t-1's prediction -- runs on stream C; the
-// partial waves of either leave SMs idle that the other fills.  Uploads of L (up to four frames ahead) and downloads
-// of ab run on two copy streams so that neither compute stream ever waits for PCIe.  L / ab may be host (pinned) or
-// device memory.
-extern "C" int dvc_colorize_clip(dvc_ctx* c, const float* L_in, int F, int H, int W, float temperature,
-                                 const float* first_last, float* ab_out, void* stream) {
-  if (!c || !L_in || !ab_out || F < 1) return c ? fail(c, DVC_ERR_ARG, "colorize_clip: bad argument") : DVC_ERR_ARG;
-  DVC_TRY(check_frame_args(c, H, W, temperature));
-  cudaStream_t s = (cudaStream_t)stream;
-  CUDA_TRY(c, cudaSetDevice(c->device));
-  DVC_TRY(clip_streams(c));
+// Per-frame stages of the clip driver around the two network phases (dvc_colorize_clip: plain copies of L and ab;
+// dvc_colorize_video_rgb8: uint8 frames in, ingest, batched post-processing, uint8 frames out).
+struct ClipStages {
+  // upload stream: frame t's half-size L into the slot Lt (the driver has made su wait until the slot is free)
+  std::function<int(int t, float* Lt, cudaStream_t su)> ingest;
+  // the half-size ab slot frame t's ColorVidNet writes; makes sc wait until the slot is free
+  std::function<int(int t, cudaStream_t sc, float** abt)> ab_slot;
+  // hands frame t's ab on once `done` (recorded on the ColorVidNet stream after frame t) has fired
+  std::function<int(int t, const float* abt, cudaEvent_t done)> egress;
+};
+
+// test.py:68-96 for one contiguous segment of F frames, starting from the previous frame's Lab in `dlast` (updated in place).
+// Frame t+1's frame-independent phase (VGG / WarpNet / correlation) runs on stream A while frame t's ColorVidNet -- which
+// needs frame t-1's prediction -- runs on stream C; the partial waves of either leave SMs idle that the other fills.
+// Ingest (up to four frames ahead) and egress run on their own streams so that neither compute stream waits for PCIe.
+static int run_clip(dvc_ctx* c, int F, int H, int W, float temperature, float* dlast, const ClipStages& st, cudaStream_t s) {
   const size_t hw = (size_t)H * W;
   const int N = (H / 4) * (W / 4);
-  void *dL, *dlast, *dab, *yrows, *simrows;
+  void *dL, *yrows, *simrows;
   DVC_TRY(get_raw(c, "clip.L", 4 * hw * 4, &dL, s));   // 4 slots
-  DVC_TRY(get_raw(c, "clip.last", 3 * hw * 4, &dlast, s));
-  DVC_TRY(get_raw(c, "clip.ab", 2 * 2 * hw * 4, &dab, s));  // 2 slots
   DVC_TRY(get_raw(c, "clip.yrows", (size_t)4 * N * 16, &yrows, s));  // 4 slots: phase A may run up to 3 frames ahead
   DVC_TRY(get_raw(c, "clip.simrows", (size_t)4 * N * 4, &simrows, s));
   const bool two_a = c->clip_astreams == 2;
   // the second phase-A stream has its own correlation workspace (sized like the first at dvc_set_exemplar time)
   if (two_a && corr_ws_reserve(&c->corr_ws2, 1, 1, N, N) != 0) return fail(c, DVC_ERR_CUDA, "colorize_clip: correlation workspace allocation failed");
-  if (first_last)
-    CUDA_TRY(c, cudaMemcpyAsync(dlast, first_last, 3 * hw * 4, cudaMemcpyDefault, s));
-  else
-    CUDA_TRY(c, cudaMemsetAsync(dlast, 0, 3 * hw * 4, s));  // test.py:80
   // Every exit below goes through the join epilogue: an error in the middle of the loop must not return while copies
-  // or kernels of earlier frames are still writing into ab_out / the slots (a retry would race with them).
+  // or kernels of earlier frames are still writing into the outputs / the slots (a retry would race with them).
   auto enqueue = [&]() -> int {
     CUDA_TRY(c, cudaEventRecord(c->evFork, s));
-    CUDA_TRY(c, cudaStreamWaitEvent(c->sA, c->evFork, 0));
-    CUDA_TRY(c, cudaStreamWaitEvent(c->sA2, c->evFork, 0));
-    CUDA_TRY(c, cudaStreamWaitEvent(c->sC, c->evFork, 0));
-    CUDA_TRY(c, cudaStreamWaitEvent(c->sU, c->evFork, 0));
-    CUDA_TRY(c, cudaStreamWaitEvent(c->sD, c->evFork, 0));
+    for (cudaStream_t si : {c->sA, c->sA2, c->sC, c->sU, c->sD, c->sP}) CUDA_TRY(c, cudaStreamWaitEvent(si, c->evFork, 0));
     for (int t = 0; t < F; ++t) {
-      const int slot = t & 1;
       float* Lt = (float*)dL + (size_t)(t & 3) * hw;
-      float* abt = (float*)dab + (size_t)slot * 2 * hw;
       float* yr = (float*)yrows + (size_t)(t & 3) * N * 4;
       float* sr = (float*)simrows + (size_t)(t & 3) * N;
       const bool odd = two_a && (t & 1);
       cudaStream_t sAt = odd ? c->sA2 : c->sA;
       // ---- upload stream: the L slot was last read by frame t-4's ColorVidNet / make_last ----
       if (t >= 4) CUDA_TRY(c, cudaStreamWaitEvent(c->sU, c->evC[(t - 4) & 3], 0));
-      CUDA_TRY(c, cudaMemcpyAsync(Lt, L_in + (size_t)t * hw, hw * 4, cudaMemcpyDefault, c->sU));
+      DVC_TRY(st.ingest(t, Lt, c->sU));
       CUDA_TRY(c, cudaEventRecord(c->evU[t & 3], c->sU));
       // ---- stream A (two of them, alternating, when clip_astreams = 2): the frame-independent phase; the reuse of the
       // warp-row slot waits for frame t-4's ColorVidNet ----
@@ -1710,32 +1719,30 @@ extern "C" int dvc_colorize_clip(dvc_ctx* c, const float* L_in, int F, int H, in
       CUDA_TRY(c, cudaEventRecord(c->evA[t & 3], sAt));
       // ---- stream C: the recurrent phase ----
       CUDA_TRY(c, cudaStreamWaitEvent(c->sC, c->evA[t & 3], 0));
-      if (t >= 2) CUDA_TRY(c, cudaStreamWaitEvent(c->sC, c->evD[(t - 2) & 3], 0));  // the ab slot has been downloaded
-      DVC_TRY(frames_phaseC(c, "clipC", Lt, yr, sr, (float*)dlast, 1, H, W, abt, c->sC));
-      launch_make_last(Lt, abt, (float*)dlast, 1, H, W, c->sC);  // test.py:96
+      float* abt = nullptr;
+      DVC_TRY(st.ab_slot(t, c->sC, &abt));
+      DVC_TRY(frames_phaseC(c, "clipC", Lt, yr, sr, dlast, 1, H, W, abt, c->sC));
+      launch_make_last(Lt, abt, dlast, 1, H, W, c->sC);  // test.py:96
       DVC_TRY(check_launch(c, "make_last"));
       CUDA_TRY(c, cudaEventRecord(c->evC[t & 3], c->sC));
-      // ---- download stream ----
-      CUDA_TRY(c, cudaStreamWaitEvent(c->sD, c->evC[t & 3], 0));
-      CUDA_TRY(c, cudaMemcpyAsync(ab_out + (size_t)t * 2 * hw, abt, 2 * hw * 4, cudaMemcpyDefault, c->sD));
-      CUDA_TRY(c, cudaEventRecord(c->evD[t & 3], c->sD));
+      DVC_TRY(st.egress(t, abt, c->evC[t & 3]));
     }
     return DVC_OK;
   };
   const int rc = enqueue();
   const std::string first_err = c->err;
-  // join: the caller's stream waits for the four internal streams, then the host waits for the caller's stream
+  // join: the caller's stream waits for the internal streams, then the host waits for the caller's stream
   bool join_ok = true;
   join_ok &= cudaEventRecord(c->evJoinA, c->sA) == cudaSuccess && cudaStreamWaitEvent(s, c->evJoinA, 0) == cudaSuccess;
   join_ok &= cudaEventRecord(c->evJoinA2, c->sA2) == cudaSuccess && cudaStreamWaitEvent(s, c->evJoinA2, 0) == cudaSuccess;
   join_ok &= cudaEventRecord(c->evJoinC, c->sC) == cudaSuccess && cudaStreamWaitEvent(s, c->evJoinC, 0) == cudaSuccess;
   join_ok &= cudaEventRecord(c->evJoinD, c->sD) == cudaSuccess && cudaStreamWaitEvent(s, c->evJoinD, 0) == cudaSuccess;
+  join_ok &= cudaEventRecord(c->evJoinP, c->sP) == cudaSuccess && cudaStreamWaitEvent(s, c->evJoinP, 0) == cudaSuccess;
   join_ok &= cudaEventRecord(c->evFork, c->sU) == cudaSuccess && cudaStreamWaitEvent(s, c->evFork, 0) == cudaSuccess;
   const cudaError_t se = cudaStreamSynchronize(s);
   if (rc != DVC_OK) {
     if (!join_ok || se != cudaSuccess) {  // could not even drain the streams: make sure nothing is in flight
-      cudaStreamSynchronize(c->sA), cudaStreamSynchronize(c->sA2), cudaStreamSynchronize(c->sC), cudaStreamSynchronize(c->sU),
-          cudaStreamSynchronize(c->sD);
+      for (cudaStream_t si : {c->sA, c->sA2, c->sC, c->sU, c->sD, c->sP}) cudaStreamSynchronize(si);
     }
     c->err = first_err;
     return rc;
@@ -1743,6 +1750,41 @@ extern "C" int dvc_colorize_clip(dvc_ctx* c, const float* L_in, int F, int H, in
   if (!join_ok) return fail(c, DVC_ERR_CUDA, "colorize_clip: joining the internal streams failed");
   if (se != cudaSuccess) return fail(c, DVC_ERR_CUDA, std::string("colorize_clip: ") + cudaGetErrorString(se));
   return DVC_OK;
+}
+
+// L / ab may be host (pinned) or device memory.
+extern "C" int dvc_colorize_clip(dvc_ctx* c, const float* L_in, int F, int H, int W, float temperature,
+                                 const float* first_last, float* ab_out, void* stream) {
+  if (!c || !L_in || !ab_out || F < 1) return c ? fail(c, DVC_ERR_ARG, "colorize_clip: bad argument") : DVC_ERR_ARG;
+  DVC_TRY(check_frame_args(c, H, W, temperature));
+  cudaStream_t s = (cudaStream_t)stream;
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  DVC_TRY(clip_streams(c));
+  const size_t hw = (size_t)H * W;
+  void *dlast, *dab;
+  DVC_TRY(get_raw(c, "clip.last", 3 * hw * 4, &dlast, s));
+  DVC_TRY(get_raw(c, "clip.ab", 2 * 2 * hw * 4, &dab, s));  // 2 slots
+  if (first_last)
+    CUDA_TRY(c, cudaMemcpyAsync(dlast, first_last, 3 * hw * 4, cudaMemcpyDefault, s));
+  else
+    CUDA_TRY(c, cudaMemsetAsync(dlast, 0, 3 * hw * 4, s));  // test.py:80
+  ClipStages st;
+  st.ingest = [&](int t, float* Lt, cudaStream_t su) -> int {
+    CUDA_TRY(c, cudaMemcpyAsync(Lt, L_in + (size_t)t * hw, hw * 4, cudaMemcpyDefault, su));
+    return DVC_OK;
+  };
+  st.ab_slot = [&](int t, cudaStream_t sc, float** abt) -> int {
+    if (t >= 2) CUDA_TRY(c, cudaStreamWaitEvent(sc, c->evD[(t - 2) & 3], 0));  // the ab slot has been downloaded
+    *abt = (float*)dab + (size_t)(t & 1) * 2 * hw;
+    return DVC_OK;
+  };
+  st.egress = [&](int t, const float* abt, cudaEvent_t done) -> int {
+    CUDA_TRY(c, cudaStreamWaitEvent(c->sD, done, 0));
+    CUDA_TRY(c, cudaMemcpyAsync(ab_out + (size_t)t * 2 * hw, abt, 2 * hw * 4, cudaMemcpyDefault, c->sD));
+    CUDA_TRY(c, cudaEventRecord(c->evD[t & 3], c->sD));
+    return DVC_OK;
+  };
+  return run_clip(c, F, H, W, temperature, (float*)dlast, st, s);
 }
 
 // ---- pre / post-processing around the nets (SURVEY.md §8f row 1) -----------------------------------------
@@ -1762,16 +1804,22 @@ extern "C" int dvc_upsample2_scaled(dvc_ctx* c, const float* dev_src, int planes
   return check_launch(c, "upsample2");
 }
 
+// rgb_from_xyz = inv(xyz_from_rgb) (skimage.color.colorconv), by the adjugate in double precision
+static void rgb_from_xyz(double inv[9]) {
+  const double a[9] = {0.412453, 0.357580, 0.180423, 0.212671, 0.715160, 0.072169, 0.019334, 0.119193, 0.950227};
+  const double det = a[0] * (a[4] * a[8] - a[5] * a[7]) - a[1] * (a[3] * a[8] - a[5] * a[6]) + a[2] * (a[3] * a[7] - a[4] * a[6]);
+  const double m[9] = {(a[4] * a[8] - a[5] * a[7]) / det, (a[2] * a[7] - a[1] * a[8]) / det, (a[1] * a[5] - a[2] * a[4]) / det,
+                       (a[5] * a[6] - a[3] * a[8]) / det, (a[0] * a[8] - a[2] * a[6]) / det, (a[2] * a[3] - a[0] * a[5]) / det,
+                       (a[3] * a[7] - a[4] * a[6]) / det, (a[1] * a[6] - a[0] * a[7]) / det, (a[0] * a[4] - a[1] * a[3]) / det};
+  for (int i = 0; i < 9; ++i) inv[i] = m[i];
+}
+
 extern "C" int dvc_lab_to_rgb8(dvc_ctx* c, const float* dev_l, const float* dev_ab, int B, int H, int W, unsigned char* dev_rgb,
                                void* stream) {
   if (!c || !dev_l || !dev_ab || !dev_rgb || B < 1 || H < 1 || W < 1) return c ? fail(c, DVC_ERR_ARG, "lab_to_rgb8: bad argument") : DVC_ERR_ARG;
   CUDA_TRY(c, cudaSetDevice(c->device));
-  // rgb_from_xyz = inv(xyz_from_rgb) (skimage.color.colorconv), by the adjugate in double precision
-  const double a[9] = {0.412453, 0.357580, 0.180423, 0.212671, 0.715160, 0.072169, 0.019334, 0.119193, 0.950227};
-  const double det = a[0] * (a[4] * a[8] - a[5] * a[7]) - a[1] * (a[3] * a[8] - a[5] * a[6]) + a[2] * (a[3] * a[7] - a[4] * a[6]);
-  const double inv[9] = {(a[4] * a[8] - a[5] * a[7]) / det, (a[2] * a[7] - a[1] * a[8]) / det, (a[1] * a[5] - a[2] * a[4]) / det,
-                         (a[5] * a[6] - a[3] * a[8]) / det, (a[0] * a[8] - a[2] * a[6]) / det, (a[2] * a[3] - a[0] * a[5]) / det,
-                         (a[3] * a[7] - a[4] * a[6]) / det, (a[1] * a[6] - a[0] * a[7]) / det, (a[0] * a[4] - a[1] * a[3]) / det};
+  double inv[9];
+  rgb_from_xyz(inv);
   launch_lab_to_rgb8(dev_l, dev_ab, dev_rgb, B, H, W, inv, (cudaStream_t)stream);
   return check_launch(c, "lab_to_rgb8");
 }
@@ -1828,34 +1876,48 @@ extern "C" int dvc_contextual_loss_forward(dvc_ctx* c, const float* dev_X, const
 }
 
 // ---- Fast Global Smoother ("WLS filter", test.py:105-112) ---------------------------------------------------------
+// weights_LUT[d] = -exp(-d / sigma_color), d = |difference of neighbouring guide pixels|: evaluated in double and rounded
+// once to the fp32 work type (the oracle does the same, so the two agree bit for bit).  Uploaded once per call.
+static int fgs_lut(dvc_ctx* c, const std::string& name, float sigma_color, float** out, cudaStream_t s) {
+  void* lut;
+  DVC_TRY(get_raw(c, name, 256 * 4, &lut, s));
+  float h_lut[256];
+  for (int d = 0; d < 256; ++d) h_lut[d] = (float)(-exp(-(double)d / (double)sigma_color));
+  CUDA_TRY(c, cudaMemcpyAsync(lut, h_lut, sizeof(h_lut), cudaMemcpyHostToDevice, s));
+  CUDA_TRY(c, cudaStreamSynchronize(s));  // h_lut lives on this stack frame
+  *out = (float*)lut;
+  return DVC_OK;
+}
+
+// F frames of P planes x [F][P][H][W] filtered in place, frame f guided by guide [f] ([F][H][W]): one launch per step
+static int fgs_run(dvc_ctx* c, const std::string& tag, const unsigned char* guide, float* x, int F, int P, int H, int W, float lambda,
+                   const float* lut, float lambda_attenuation, int num_iter, cudaStream_t s) {
+  const size_t hw = (size_t)H * W;
+  void *Ch, *Cv, *D;
+  DVC_TRY(get_raw(c, tag + ".Ch", (size_t)F * hw * 4, &Ch, s));
+  DVC_TRY(get_raw(c, tag + ".Cv", (size_t)F * hw * 4, &Cv, s));
+  DVC_TRY(get_raw(c, tag + ".D", (size_t)F * P * hw * 4, &D, s));
+  launch_fgs_weights(guide, lut, (float*)Ch, (float*)Cv, F, H, W, s);
+  DVC_TRY(check_launch(c, "fgs_weights"));
+  float lam = lambda;
+  for (int n = 0; n < num_iter; ++n) {
+    launch_fgs_horizontal(x, (const float*)Ch, (float*)D, F * P, P, H, W, lam, s);
+    launch_fgs_vertical(x, (const float*)Cv, (float*)D, F * P, P, H, W, lam, s);
+    lam *= lambda_attenuation;
+  }
+  return check_launch(c, "fgs");
+}
+
 extern "C" int dvc_fgs_filter(dvc_ctx* c, const unsigned char* dev_guide, const float* dev_src, int planes, int H, int W, float lambda,
                               float sigma_color, float lambda_attenuation, int num_iter, float* dev_dst, void* stream) {
   if (!c || !dev_guide || !dev_src || !dev_dst || planes < 1 || H < 2 || W < 2) return c ? fail(c, DVC_ERR_ARG, "fgs_filter: bad argument") : DVC_ERR_ARG;
   if (!(lambda >= 0.f) || !(sigma_color > 0.f) || num_iter < 1 || !(lambda_attenuation > 0.f)) return fail(c, DVC_ERR_ARG, "fgs_filter: bad parameter");
   cudaStream_t s = (cudaStream_t)stream;
   CUDA_TRY(c, cudaSetDevice(c->device));
-  const size_t hw = (size_t)H * W;
-  void *lut, *Ch, *Cv, *D;
-  DVC_TRY(get_raw(c, "fgs.lut", 256 * 4, &lut, s));
-  DVC_TRY(get_raw(c, "fgs.Ch", hw * 4, &Ch, s));
-  DVC_TRY(get_raw(c, "fgs.Cv", hw * 4, &Cv, s));
-  DVC_TRY(get_raw(c, "fgs.D", (size_t)planes * hw * 4, &D, s));
-  // weights_LUT[d] = -exp(-d / sigma_color), d = |difference of neighbouring guide pixels|: evaluated in double and
-  // rounded once to the fp32 work type (the oracle does the same, so the two agree bit for bit)
-  float h_lut[256];
-  for (int d = 0; d < 256; ++d) h_lut[d] = (float)(-exp(-(double)d / (double)sigma_color));
-  CUDA_TRY(c, cudaMemcpyAsync(lut, h_lut, sizeof(h_lut), cudaMemcpyHostToDevice, s));
-  CUDA_TRY(c, cudaStreamSynchronize(s));  // h_lut lives on this stack frame
-  launch_fgs_weights(dev_guide, (const float*)lut, (float*)Ch, (float*)Cv, H, W, s);
-  DVC_TRY(check_launch(c, "fgs_weights"));
-  if (dev_dst != dev_src) CUDA_TRY(c, cudaMemcpyAsync(dev_dst, dev_src, (size_t)planes * hw * 4, cudaMemcpyDeviceToDevice, s));
-  float lam = lambda;
-  for (int n = 0; n < num_iter; ++n) {
-    launch_fgs_horizontal(dev_dst, (const float*)Ch, (float*)D, planes, H, W, lam, s);
-    launch_fgs_vertical(dev_dst, (const float*)Cv, (float*)D, planes, H, W, lam, s);
-    lam *= lambda_attenuation;
-  }
-  return check_launch(c, "fgs");
+  float* lut;
+  DVC_TRY(fgs_lut(c, "fgs.lut", sigma_color, &lut, s));
+  if (dev_dst != dev_src) CUDA_TRY(c, cudaMemcpyAsync(dev_dst, dev_src, (size_t)planes * H * W * 4, cudaMemcpyDeviceToDevice, s));
+  return fgs_run(c, "fgs", dev_guide, dev_dst, 1, planes, H, W, lambda, lut, lambda_attenuation, num_iter, s);
 }
 
 extern "C" int dvc_l_to_guide8(dvc_ctx* c, const float* dev_l, int H, int W, unsigned char* dev_guide, void* stream) {
@@ -1876,17 +1938,16 @@ static void gaussian_taps(double sigma, std::vector<double>* w, int* radius) {  
   *radius = r;
 }
 
-extern "C" int dvc_resize_antialias_crop_rgb8(dvc_ctx* c, const unsigned char* dev_src, int Hs, int Ws, int Hr, int Wr, int oy, int ox,
-                                              unsigned char* dev_dst, int Ho, int Wo, void* stream) {
-  if (!c || !dev_src || !dev_dst || Hs < 1 || Ws < 1 || Hr < 1 || Wr < 1 || Ho < 1 || Wo < 1)
-    return c ? fail(c, DVC_ERR_ARG, "resize_antialias_crop: bad argument") : DVC_ERR_ARG;
-  cudaStream_t s = (cudaStream_t)stream;
-  CUDA_TRY(c, cudaSetDevice(c->device));
-  const size_t n = (size_t)Hs * Ws * 3;
-  void *f0, *f1, *taps;
-  DVC_TRY(get_raw(c, "rs.f0", n * 8, &f0, s));
-  DVC_TRY(get_raw(c, "rs.f1", n * 8, &f1, s));
-  DVC_TRY(get_raw(c, "rs.taps", 8192 * 8, &taps, s));
+// skimage.transform.resize's anti-aliasing Gaussians for an Hs x Ws -> Hr x Wr resize on the device: wy (2 ry + 1 taps),
+// wx (2 rx + 1) and, at index 8191, a lone tap of weight 1 that converts uint8 -> float64 when the y axis needs no filter.
+// Uploaded once per call (the host vectors live on this stack frame: the stream is synchronised).
+struct ResizeTaps {
+  const double *wy = nullptr, *wx = nullptr;
+  int ry = 0, rx = 0;
+};
+static int resize_taps(dvc_ctx* c, const std::string& name, int Hs, int Ws, int Hr, int Wr, ResizeTaps* tp, cudaStream_t s) {
+  void* taps;
+  DVC_TRY(get_raw(c, name, 8192 * 8, &taps, s));
   // skimage.transform.resize: sigma = max(0, (in / out - 1) / 2) per axis, applied axis 0 first (scipy.ndimage.gaussian_filter)
   const double sy = fmax(0.0, ((double)Hs / Hr - 1.0) / 2.0), sx = fmax(0.0, ((double)Ws / Wr - 1.0) / 2.0);
   std::vector<double> wy, wx;
@@ -1894,26 +1955,175 @@ extern "C" int dvc_resize_antialias_crop_rgb8(dvc_ctx* c, const unsigned char* d
   if (sy > 1e-15) gaussian_taps(sy, &wy, &ry);
   if (sx > 1e-15) gaussian_taps(sx, &wx, &rx);
   if (wy.size() + wx.size() > 8192) return fail(c, DVC_ERR_SHAPE, "resize_antialias_crop: down-scaling factor too large");
+  const double one = 1.0;
   if (!wy.empty()) CUDA_TRY(c, cudaMemcpyAsync(taps, wy.data(), wy.size() * 8, cudaMemcpyHostToDevice, s));
   if (!wx.empty()) CUDA_TRY(c, cudaMemcpyAsync((double*)taps + wy.size(), wx.data(), wx.size() * 8, cudaMemcpyHostToDevice, s));
-  CUDA_TRY(c, cudaStreamSynchronize(s));  // the tap vectors live on this stack frame
-  // image as float64 [Hs][Ws][3]; a zero-radius "filter" (one tap of weight 1) converts uint8 -> float64 when an axis needs none
-  const double one = 1.0;
+  if (wy.empty()) CUDA_TRY(c, cudaMemcpyAsync((double*)taps + 8191, &one, 8, cudaMemcpyHostToDevice, s));
+  CUDA_TRY(c, cudaStreamSynchronize(s));
+  tp->wy = wy.empty() ? (double*)taps + 8191 : (double*)taps, tp->ry = ry;
+  tp->wx = wx.empty() ? nullptr : (double*)taps + wy.size(), tp->rx = rx;
+  return DVC_OK;
+}
+
+// F uint8 frames [F][Hs][Ws][3] -> the anti-aliased float64 frames [F][Hs][Ws][3] (the Gaussian along y, then along x)
+static int antialias_f64(dvc_ctx* c, const std::string& tag, const unsigned char* src, int F, int Hs, int Ws, const ResizeTaps& tp,
+                         double** out, cudaStream_t s) {
+  const size_t n = (size_t)F * Hs * Ws * 3;
+  void *f0, *f1;
+  DVC_TRY(get_raw(c, tag + ".f0", n * 8, &f0, s));
+  DVC_TRY(get_raw(c, tag + ".f1", n * 8, &f1, s));
   double* cur = (double*)f0;
   double* nxt = (double*)f1;
-  if (wy.empty()) {
-    CUDA_TRY(c, cudaMemcpyAsync((double*)taps + 8191, &one, 8, cudaMemcpyHostToDevice, s));
-    CUDA_TRY(c, cudaStreamSynchronize(s));
-    launch_gauss_axis_u8(dev_src, cur, (double*)taps + 8191, 0, 1, Hs, Ws * 3, s);
-  } else {
-    launch_gauss_axis_u8(dev_src, cur, (double*)taps, ry, 1, Hs, Ws * 3, s);
-  }
-  if (!wx.empty()) {
-    launch_gauss_axis_f64(cur, nxt, (double*)taps + wy.size(), rx, (size_t)Hs, Ws, 3, s);
+  launch_gauss_axis_u8(src, cur, tp.wy, tp.ry, (size_t)F, Hs, Ws * 3, s);
+  if (tp.wx) {
+    launch_gauss_axis_f64(cur, nxt, tp.wx, tp.rx, (size_t)F * Hs, Ws, 3, s);
     std::swap(cur, nxt);
   }
+  *out = cur;
+  return check_launch(c, "antialias");
+}
+
+static bool bad_geometry(int Hs, int Ws, int Hr, int Wr, int Ho, int Wo) { return Hs < 1 || Ws < 1 || Hr < 1 || Wr < 1 || Ho < 1 || Wo < 1; }
+
+extern "C" int dvc_resize_antialias_crop_rgb8(dvc_ctx* c, const unsigned char* dev_src, int Hs, int Ws, int Hr, int Wr, int oy, int ox,
+                                              unsigned char* dev_dst, int Ho, int Wo, void* stream) {
+  if (!c || !dev_src || !dev_dst || bad_geometry(Hs, Ws, Hr, Wr, Ho, Wo))
+    return c ? fail(c, DVC_ERR_ARG, "resize_antialias_crop: bad argument") : DVC_ERR_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  ResizeTaps tp;
+  DVC_TRY(resize_taps(c, "rs.taps", Hs, Ws, Hr, Wr, &tp, s));
+  double* cur;
+  DVC_TRY(antialias_f64(c, "rs", dev_src, 1, Hs, Ws, tp, &cur, s));
   launch_zoom_crop(cur, Hs, Ws, Hr, Wr, oy, ox, dev_dst, Ho, Wo, s);
   return check_launch(c, "resize_antialias_crop");
+}
+
+// ---- whole frames in, whole frames out ---------------------------------------------------------------------------------
+static int ingest_enqueue(dvc_ctx* c, const std::string& tag, const unsigned char* src, int F, int Hs, int Ws, int Hr, int Wr, int oy,
+                          int ox, int Ho, int Wo, const ResizeTaps& tp, float* l, float* l_half, cudaStream_t s) {
+  double* cur;
+  DVC_TRY(antialias_f64(c, tag, src, F, Hs, Ws, tp, &cur, s));
+  launch_ingest_l(cur, F, Hs, Ws, Hr, Wr, oy, ox, l, Ho, Wo, s);
+  launch_resize_half(l, l_half, F, Ho, Wo, s);  // test.py:71
+  return check_launch(c, "ingest");
+}
+
+static int postprocess_enqueue(dvc_ctx* c, const std::string& tag, const float* l, const float* ab_half, int F, int Ho, int Wo, int wls,
+                               float lambda, const float* lut, unsigned char* rgb, cudaStream_t s) {
+  const size_t hw = (size_t)Ho * Wo;
+  void *up, *guide;
+  DVC_TRY(get_raw(c, tag + ".up", (size_t)F * 2 * hw * 4, &up, s));
+  launch_upsample2(ab_half, (float*)up, F * 2, Ho / 2, Wo / 2, 1.25f, s);  // test.py:100-102
+  if (wls) {                                                              // test.py:105-112
+    DVC_TRY(get_raw(c, tag + ".guide", (size_t)F * hw, &guide, s));
+    launch_l_to_guide8(l, (unsigned char*)guide, (size_t)F * hw, s);
+    DVC_TRY(fgs_run(c, tag, (const unsigned char*)guide, (float*)up, F, 2, Ho, Wo, lambda, lut, 0.25f, 3, s));
+  }
+  double inv[9];
+  rgb_from_xyz(inv);
+  launch_lab_to_rgb8(l, (const float*)up, rgb, F, Ho, Wo, inv, s);  // test.py:116-119
+  return check_launch(c, "postprocess");
+}
+
+static bool bad_out_size(int Ho, int Wo) { return Ho < 2 || Wo < 2 || (Ho & 1) || (Wo & 1); }
+static int check_wls(dvc_ctx* c, float lambda, float sigma_color) {
+  if (!(lambda >= 0.f) || !(sigma_color > 0.f)) return fail(c, DVC_ERR_ARG, "WLS filter: lambda must be >= 0 and sigma_color > 0");
+  return DVC_OK;
+}
+
+extern "C" int dvc_ingest_rgb8(dvc_ctx* c, const unsigned char* dev_src, int F, int Hs, int Ws, int Hr, int Wr, int oy, int ox, int Ho,
+                               int Wo, float* dev_l, float* dev_l_half, void* stream) {
+  if (!c || !dev_src || !dev_l || !dev_l_half || F < 1 || bad_geometry(Hs, Ws, Hr, Wr, Ho, Wo))
+    return c ? fail(c, DVC_ERR_ARG, "ingest_rgb8: bad argument") : DVC_ERR_ARG;
+  if (bad_out_size(Ho, Wo)) return fail(c, DVC_ERR_SHAPE, "ingest_rgb8: Ho and Wo must be even");
+  cudaStream_t s = (cudaStream_t)stream;
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  ResizeTaps tp;
+  DVC_TRY(resize_taps(c, "ing.taps", Hs, Ws, Hr, Wr, &tp, s));
+  return ingest_enqueue(c, "ing", dev_src, F, Hs, Ws, Hr, Wr, oy, ox, Ho, Wo, tp, dev_l, dev_l_half, s);
+}
+
+extern "C" int dvc_postprocess_rgb8(dvc_ctx* c, const float* dev_l, const float* dev_ab_half, int F, int Ho, int Wo, int wls, float lambda,
+                                    float sigma_color, unsigned char* dev_rgb, void* stream) {
+  if (!c || !dev_l || !dev_ab_half || !dev_rgb || F < 1) return c ? fail(c, DVC_ERR_ARG, "postprocess_rgb8: bad argument") : DVC_ERR_ARG;
+  if (bad_out_size(Ho, Wo)) return fail(c, DVC_ERR_SHAPE, "postprocess_rgb8: Ho and Wo must be even");
+  if (wls) DVC_TRY(check_wls(c, lambda, sigma_color));
+  cudaStream_t s = (cudaStream_t)stream;
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  float* lut = nullptr;
+  if (wls) DVC_TRY(fgs_lut(c, "post.lut", sigma_color, &lut, s));
+  return postprocess_enqueue(c, "post", dev_l, dev_ab_half, F, Ho, Wo, wls, lambda, lut, dev_rgb, s);
+}
+
+// The clip driver with uint8 frames on both ends.  Rings (device memory depends on the frame sizes and G only):
+//   source frame  1 slot  (H2D and ingest are ordered on the upload stream)
+//   full-size L   2G slots  } batch b of G frames uses slot half b & 1; written by ingest / ColorVidNet, read by the
+//   half-size ab  2G slots  } batch's post-processing, reused by batch b + 2 after evP[b & 1]
+//   RGB           G slots   (post-processing and the download are ordered on the post stream)
+extern "C" int dvc_colorize_video_rgb8(dvc_ctx* c, const unsigned char* host_src, int K, int Hs, int Ws, int Hr, int Wr, int oy, int ox,
+                                       int Ho, int Wo, float temperature, int wls, float lambda, float sigma_color, int continue_clip,
+                                       unsigned char* host_dst, void* stream) {
+  if (!c || !host_src || !host_dst || K < 1 || bad_geometry(Hs, Ws, Hr, Wr, Ho, Wo))
+    return c ? fail(c, DVC_ERR_ARG, "colorize_video_rgb8: bad argument") : DVC_ERR_ARG;
+  if (bad_out_size(Ho, Wo)) return fail(c, DVC_ERR_SHAPE, "colorize_video_rgb8: Ho and Wo must be even");
+  if (wls) DVC_TRY(check_wls(c, lambda, sigma_color));
+  const int H = Ho / 2, W = Wo / 2;
+  DVC_TRY(check_frame_args(c, H, W, temperature));
+  if (continue_clip && (c->vid_ex_version != c->ex_version || c->vid_Ho != Ho || c->vid_Wo != Wo))
+    return fail(c, DVC_ERR_STATE, "colorize_video_rgb8: nothing to continue (no earlier call against this exemplar at this size)");
+  cudaStream_t s = (cudaStream_t)stream;
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  DVC_TRY(clip_streams(c));
+  const int G = c->video_batch;
+  const size_t hw = (size_t)H * W, HW = (size_t)Ho * Wo, src_bytes = (size_t)Hs * Ws * 3;
+  void *dlast, *dsrc, *dLf, *dab, *drgb;
+  DVC_TRY(get_raw(c, "vid.last", 3 * hw * 4, &dlast, s));
+  DVC_TRY(get_raw(c, "vid.src", src_bytes, &dsrc, s));
+  DVC_TRY(get_raw(c, "vid.Lfull", (size_t)2 * G * HW * 4, &dLf, s));
+  DVC_TRY(get_raw(c, "vid.ab", (size_t)2 * G * 2 * hw * 4, &dab, s));
+  DVC_TRY(get_raw(c, "vid.rgb", (size_t)G * HW * 3, &drgb, s));
+  {  // post-processing work buffers at their full batch size now: growing one inside the frame loop would cudaFree it
+    void* p;
+    DVC_TRY(get_raw(c, "vid.up", (size_t)G * 2 * HW * 4, &p, s));
+    DVC_TRY(get_raw(c, "vid.guide", (size_t)G * HW, &p, s));
+    DVC_TRY(get_raw(c, "vid.Ch", (size_t)G * HW * 4, &p, s));
+    DVC_TRY(get_raw(c, "vid.Cv", (size_t)G * HW * 4, &p, s));
+    DVC_TRY(get_raw(c, "vid.D", (size_t)G * 2 * HW * 4, &p, s));
+  }
+  ResizeTaps tp;
+  DVC_TRY(resize_taps(c, "vid.taps", Hs, Ws, Hr, Wr, &tp, s));
+  float* lut = nullptr;
+  if (wls) DVC_TRY(fgs_lut(c, "vid.lut", sigma_color, &lut, s));
+  c->vid_ex_version = -1;  // valid again only once this call has succeeded
+  if (!continue_clip) CUDA_TRY(c, cudaMemsetAsync(dlast, 0, 3 * hw * 4, s));  // test.py:80
+  float* Lfull = (float*)dLf;
+  float* ab = (float*)dab;
+  ClipStages st;
+  st.ingest = [&](int t, float* Lt, cudaStream_t su) -> int {
+    if (t >= 2 * G) CUDA_TRY(c, cudaStreamWaitEvent(su, c->evP[(t / G) & 1], 0));  // batch t / G - 2 is post-processed
+    CUDA_TRY(c, cudaMemcpyAsync(dsrc, host_src + (size_t)t * src_bytes, src_bytes, cudaMemcpyDefault, su));
+    return ingest_enqueue(c, "vid", (const unsigned char*)dsrc, 1, Hs, Ws, Hr, Wr, oy, ox, Ho, Wo, tp, Lfull + (size_t)(t % (2 * G)) * HW,
+                          Lt, su);
+  };
+  st.ab_slot = [&](int t, cudaStream_t sc, float** abt) -> int {
+    if (t >= 2 * G) CUDA_TRY(c, cudaStreamWaitEvent(sc, c->evP[(t / G) & 1], 0));
+    *abt = ab + (size_t)(t % (2 * G)) * 2 * hw;
+    return DVC_OK;
+  };
+  st.egress = [&](int t, const float*, cudaEvent_t done) -> int {
+    if (t % G != G - 1 && t != K - 1) return DVC_OK;  // post-processing runs once per batch
+    const int n = t % G + 1, t0 = t + 1 - n, slot = t0 % (2 * G);
+    CUDA_TRY(c, cudaStreamWaitEvent(c->sP, done, 0));
+    DVC_TRY(postprocess_enqueue(c, "vid", Lfull + (size_t)slot * HW, ab + (size_t)slot * 2 * hw, n, Ho, Wo, wls, lambda, lut,
+                                (unsigned char*)drgb, c->sP));
+    CUDA_TRY(c, cudaMemcpyAsync(host_dst + (size_t)t0 * HW * 3, drgb, (size_t)n * HW * 3, cudaMemcpyDefault, c->sP));
+    CUDA_TRY(c, cudaEventRecord(c->evP[(t / G) & 1], c->sP));
+    return DVC_OK;
+  };
+  DVC_TRY(run_clip(c, K, H, W, temperature, (float*)dlast, st, s));
+  c->vid_ex_version = c->ex_version, c->vid_Ho = Ho, c->vid_Wo = Wo;
+  return DVC_OK;
 }
 
 // ---- exemplar operands for the NCCL broadcast -----------------------------------------------------

@@ -69,6 +69,29 @@ __device__ __forceinline__ void block_amax_commit(float amax, ScaleCell* cell, f
     if (m > 0.f) atomicMax(&cell->amax_bits, __float_as_uint(m));
   }
 }
+// util_distortion.py:18-23 -> skimage.color.rgb2lab of one sRGB uint8 pixel in float64, then ToTensor (.float()) and
+// Normalize (L - 50).  Shared by rgb8_to_lab_kernel and the fused frame ingest, which must agree bit for bit: keep the
+// expressions here, in one place, so the compiler contracts them the same way in both.
+__device__ __forceinline__ void rgb8_to_lab_px(const unsigned char px[3], float* L_out, float* A_out, float* B_out) {
+  double c[3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    const double v = (double)px[k] / 255.0;
+    c[k] = v > 0.04045 ? pow((v + 0.055) / 1.055, 2.4) : v / 12.92;
+  }
+  const double M[9] = {0.412453, 0.357580, 0.180423, 0.212671, 0.715160, 0.072169, 0.019334, 0.119193, 0.950227};
+  const double white[3] = {0.95047, 1.0, 1.08883};
+  double f[3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    const double t = (c[0] * M[k * 3 + 0] + c[1] * M[k * 3 + 1] + c[2] * M[k * 3 + 2]) / white[k];
+    f[k] = t > 0.008856 ? cbrt(t) : 7.787 * t + 16.0 / 116.0;
+  }
+  const float L = (float)(116.0 * f[1] - 16.0), A = (float)(500.0 * (f[0] - f[1])), Bq = (float)(200.0 * (f[1] - f[2]));
+  *L_out = L - 50.0f;
+  *A_out = A;
+  *B_out = Bq;
+}
 #endif
 
 struct Act {
@@ -239,9 +262,11 @@ void launch_lab_to_rgb8(const float* l, const float* ab, unsigned char* rgb, int
                         cudaStream_t s);
 
 // Fast Global Smoother (test.py:105-112) and the CenterPad resize (util_distortion.py:217-258): prepost.cu
-void launch_fgs_weights(const unsigned char* guide, const float* lut, float* Ch, float* Cv, int H, int W, cudaStream_t s);
-void launch_fgs_horizontal(float* cur, const float* Ch, float* D, int planes, int H, int W, float lam, cudaStream_t s);
-void launch_fgs_vertical(float* cur, const float* Cv, float* D, int planes, int H, int W, float lam, cudaStream_t s);
+// F frames: guides [F][H][W] -> weights [F][H][W]; the sweeps filter `planes` planes in place, every `ppg` consecutive planes
+// guided by the weights of one frame
+void launch_fgs_weights(const unsigned char* guide, const float* lut, float* Ch, float* Cv, int F, int H, int W, cudaStream_t s);
+void launch_fgs_horizontal(float* cur, const float* Ch, float* D, int planes, int ppg, int H, int W, float lam, cudaStream_t s);
+void launch_fgs_vertical(float* cur, const float* Cv, float* D, int planes, int ppg, int H, int W, float lam, cudaStream_t s);
 void launch_l_to_guide8(const float* l, unsigned char* g, size_t n, cudaStream_t s);
 void launch_gauss_axis_u8(const unsigned char* src, double* dst, const double* w, int radius, size_t n_outer, int len, int inner,
                           cudaStream_t s);
@@ -249,6 +274,8 @@ void launch_gauss_axis_f64(const double* src, double* dst, const double* w, int 
                            cudaStream_t s);
 void launch_zoom_crop(const double* src, int Hs, int Ws, int Hr, int Wr, int oy, int ox, unsigned char* dst, int Ho, int Wo,
                       cudaStream_t s);
+// F anti-aliased float64 frames [F][Hs][Ws][3] -> zoom + crop / pad -> uint8 -> centred L [F][Ho][Wo] in one pass
+void launch_ingest_l(const double* src, int F, int Hs, int Ws, int Hr, int Wr, int oy, int ox, float* l, int Ho, int Wo, cudaStream_t s);
 
 int64_t launch_counter_add(int64_t n);  // global launch counter (introspection)
 

@@ -749,22 +749,10 @@ namespace {
 __global__ void __launch_bounds__(256) rgb8_to_lab_kernel(const unsigned char* __restrict__ rgb, float* __restrict__ lab, int HW) {
   const int b = blockIdx.y;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < HW; i += gridDim.x * blockDim.x) {
-    double c[3];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-      const double v = (double)rgb[((size_t)b * HW + i) * 3 + k] / 255.0;
-      c[k] = v > 0.04045 ? pow((v + 0.055) / 1.055, 2.4) : v / 12.92;
-    }
-    const double M[9] = {0.412453, 0.357580, 0.180423, 0.212671, 0.715160, 0.072169, 0.019334, 0.119193, 0.950227};
-    const double white[3] = {0.95047, 1.0, 1.08883};
-    double f[3];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-      const double t = (c[0] * M[k * 3 + 0] + c[1] * M[k * 3 + 1] + c[2] * M[k * 3 + 2]) / white[k];
-      f[k] = t > 0.008856 ? cbrt(t) : 7.787 * t + 16.0 / 116.0;
-    }
-    const float L = (float)(116.0 * f[1] - 16.0), A = (float)(500.0 * (f[0] - f[1])), Bq = (float)(200.0 * (f[1] - f[2]));
-    lab[((size_t)b * 3 + 0) * HW + i] = L - 50.0f;
+    const unsigned char px[3] = {rgb[((size_t)b * HW + i) * 3 + 0], rgb[((size_t)b * HW + i) * 3 + 1], rgb[((size_t)b * HW + i) * 3 + 2]};
+    float L, A, Bq;
+    rgb8_to_lab_px(px, &L, &A, &Bq);
+    lab[((size_t)b * 3 + 0) * HW + i] = L;
     lab[((size_t)b * 3 + 1) * HW + i] = A;
     lab[((size_t)b * 3 + 2) * HW + i] = Bq;
   }

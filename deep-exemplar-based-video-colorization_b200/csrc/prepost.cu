@@ -25,11 +25,13 @@ namespace {
 
 // ------------------------------------------------------------------------------------------------ FGS
 // C_h(i, j) = -w(g(i, j), g(i, j+1)), 0 in the last column; C_v(i, j) = -w(g(i, j), g(i+1, j)), 0 in the last row.
+// F frames: guides [F][H][W] -> weights [F][H][W].
 __global__ void __launch_bounds__(256) fgs_weights_kernel(const unsigned char* __restrict__ g, const float* __restrict__ lut,
-                                                          float* __restrict__ Ch, float* __restrict__ Cv, int H, int W) {
-  const int n = H * W;
-  for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
-    const int i = p / W, j = p - i * W;
+                                                          float* __restrict__ Ch, float* __restrict__ Cv, int F, int H, int W) {
+  const size_t hw = (size_t)H * W, n = (size_t)F * hw;
+  for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (size_t)gridDim.x * blockDim.x) {
+    const int q = (int)(p % hw);
+    const int i = q / W, j = q - i * W;
     const int c = g[p];
     Ch[p] = (j + 1 < W) ? __ldg(lut + abs(c - (int)g[p + 1])) : 0.f;
     Cv[p] = (i + 1 < H) ? __ldg(lut + abs(c - (int)g[p + W])) : 0.f;
@@ -41,15 +43,17 @@ __global__ void __launch_bounds__(256) fgs_weights_kernel(const unsigned char* _
 //   forward : denom_j = (1 - lam C_{j-1} - lam C_j) - lam C_{j-1} * D_{j-1};  D_j = lam C_j / denom_j;
 //             u_j = (u_j - lam C_{j-1} u_{j-1}) / denom_j
 //   backward: u_j = u_j - D_j u_{j+1}
-// Vertical sweep: thread = (plane, column), adjacent threads touch adjacent addresses (coalesced).
+// Both sweeps take `planes` planes of which every `ppg` consecutive ones share one guide (plane pl uses the weights of
+// frame pl / ppg): one launch covers all planes of all frames.
+// Vertical sweep: thread = (plane, column), adjacent threads touch adjacent addresses (coalesced); one grid row per frame.
 __global__ void __launch_bounds__(128) fgs_vertical_kernel(float* __restrict__ cur, const float* __restrict__ Cv, float* __restrict__ D,
-                                                           int planes, int H, int W, float lam) {
-  const int t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= planes * W) return;
-  const int pl = t / W, x = t - pl * W;
+                                                           int ppg, int H, int W, float lam) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;  // blockIdx.y = frame
+  if (t >= ppg * W) return;
+  const int pl = blockIdx.y * ppg + t / W, x = t % W;
   float* u = cur + (size_t)pl * H * W + x;
   float* d = D + (size_t)pl * H * W + x;
-  const float* c = Cv + x;
+  const float* c = Cv + (size_t)blockIdx.y * H * W + x;
   float cprev = __fmul_rn(lam, c[0]);
   float denom = __fsub_rn(1.f, cprev);
   float dprev = __fdiv_rn(cprev, denom);
@@ -73,7 +77,7 @@ __global__ void __launch_bounds__(128) fgs_vertical_kernel(float* __restrict__ c
 // that are moved between global and shared memory with coalesced row accesses (a thread per row reading its own row
 // directly would touch one sector per element).
 __global__ void __launch_bounds__(32) fgs_horizontal_kernel(float* __restrict__ cur, const float* __restrict__ Ch, float* __restrict__ D,
-                                                            int planes, int H, int W, float lam) {
+                                                            int planes, int ppg, int H, int W, float lam) {
   __shared__ float su[32][33], sc[32][33], sd[32][33];
   const int lane = threadIdx.x;
   const int groups = (H + 31) / 32;
@@ -81,7 +85,7 @@ __global__ void __launch_bounds__(32) fgs_horizontal_kernel(float* __restrict__ 
   const int nrows = min(32, H - r0);
   float* ub = cur + ((size_t)pl * H + r0) * W;
   float* db = D + ((size_t)pl * H + r0) * W;
-  const float* cb = Ch + (size_t)r0 * W;
+  const float* cb = Ch + ((size_t)(pl / ppg) * H + r0) * W;
   float cprev = 0.f, dprev = 0.f, uprev = 0.f;
   for (int x0 = 0; x0 < W; x0 += 32) {
     const int nx = min(32, W - x0);
@@ -170,9 +174,29 @@ __global__ void __launch_bounds__(256) gauss_axis_kernel(const TIn* __restrict__
   }
 }
 
-// scipy.ndimage.zoom(order=1, mode="mirror", grid_mode=True) of a [Hs][Ws][3] float64 image to [Hr][Wr], truncated to
-// uint8 (ndarray.astype(np.uint8) of in-range values), then CenterPad's centred crop (offset oy, ox) / zero pad into
-// the [Ho][Wo][3] output.
+// scipy.ndimage.zoom(order=1, mode="mirror", grid_mode=True) of a [Hs][Ws][3] float64 image to [Hr][Wr], channel ch of
+// resized pixel (yr, xr), truncated to uint8 (ndarray.astype(np.uint8) of in-range values).
+__device__ __forceinline__ unsigned char zoom_px(const double* __restrict__ src, int Hs, int Ws, int Hr, int Wr, int yr, int xr, int ch) {
+  // grid_mode: pixel centres align, in = (out + 0.5) * (in_len / out_len) - 0.5
+  // (separately rounded operations throughout: see gauss_axis_kernel)
+  const double cy = __dsub_rn(__dmul_rn(__dadd_rn((double)yr, 0.5), __ddiv_rn((double)Hs, (double)Hr)), 0.5);
+  const double cx = __dsub_rn(__dmul_rn(__dadd_rn((double)xr, 0.5), __ddiv_rn((double)Ws, (double)Wr)), 0.5);
+  const double fy = floor(cy), fx = floor(cx);
+  const double ty = __dsub_rn(cy, fy), tx = __dsub_rn(cx, fx);
+  const int y0 = mirror_idx((int)fy, Hs), y1 = mirror_idx((int)fy + 1, Hs);
+  const int x0 = mirror_idx((int)fx, Ws), x1 = mirror_idx((int)fx + 1, Ws);
+  const double v00 = src[((size_t)y0 * Ws + x0) * 3 + ch], v01 = src[((size_t)y0 * Ws + x1) * 3 + ch];
+  const double v10 = src[((size_t)y1 * Ws + x0) * 3 + ch], v11 = src[((size_t)y1 * Ws + x1) * 3 + ch];
+  // scipy (ni_interpolation.c) sums the 2 x 2 neighbourhood, row-major, each term ((value * wy) * wx)
+  const double wy0 = __dsub_rn(1.0, ty), wx0 = __dsub_rn(1.0, tx);
+  double v = __dmul_rn(__dmul_rn(v00, wy0), wx0);
+  v = __dadd_rn(v, __dmul_rn(__dmul_rn(v01, wy0), tx));
+  v = __dadd_rn(v, __dmul_rn(__dmul_rn(v10, ty), wx0));
+  v = __dadd_rn(v, __dmul_rn(__dmul_rn(v11, ty), tx));
+  return (unsigned char)fmin(fmax(trunc(v), 0.0), 255.0);
+}
+
+// zoom_px, then CenterPad's centred crop (offset oy, ox) / zero pad into the [Ho][Wo][3] output.
 __global__ void __launch_bounds__(256) zoom_crop_kernel(const double* __restrict__ src, int Hs, int Ws, int Hr, int Wr, int oy, int ox,
                                                         unsigned char* __restrict__ dst, int Ho, int Wo) {
   const size_t total = (size_t)Ho * Wo * 3;
@@ -181,27 +205,29 @@ __global__ void __launch_bounds__(256) zoom_crop_kernel(const double* __restrict
     const size_t t = idx / 3;
     const int xo = (int)(t % Wo), yo = (int)(t / Wo);
     const int yr = yo + oy, xr = xo + ox;  // position in the resized image
-    unsigned char out = 0;
+    dst[idx] = (yr >= 0 && yr < Hr && xr >= 0 && xr < Wr) ? zoom_px(src, Hs, Ws, Hr, Wr, yr, xr, ch) : 0;
+  }
+}
+
+// The frame ingest of test.py:44-46 after the anti-aliasing Gaussians, for F frames [F][Hs][Ws][3] float64: zoom + crop /
+// pad (zoom_crop_kernel) -> sRGB uint8 -> Lab (rgb8_to_lab_px) -> centred L [F][Ho][Wo].  The uint8 pixel never leaves
+// registers; a/b are not needed by the networks' input and are not written.
+__global__ void __launch_bounds__(256) ingest_l_kernel(const double* __restrict__ src, int F, int Hs, int Ws, int Hr, int Wr, int oy,
+                                                       int ox, float* __restrict__ l, int Ho, int Wo) {
+  const size_t hw = (size_t)Ho * Wo, total = (size_t)F * hw;
+  for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+    const size_t f = idx / hw, q = idx - f * hw;
+    const int xo = (int)(q % Wo), yo = (int)(q / Wo);
+    const int yr = yo + oy, xr = xo + ox;
+    const double* fs = src + f * (size_t)Hs * Ws * 3;
+    unsigned char px[3] = {0, 0, 0};
     if (yr >= 0 && yr < Hr && xr >= 0 && xr < Wr) {
-      // grid_mode: pixel centres align, in = (out + 0.5) * (in_len / out_len) - 0.5
-      // (separately rounded operations throughout: see gauss_axis_kernel)
-      const double cy = __dsub_rn(__dmul_rn(__dadd_rn((double)yr, 0.5), __ddiv_rn((double)Hs, (double)Hr)), 0.5);
-      const double cx = __dsub_rn(__dmul_rn(__dadd_rn((double)xr, 0.5), __ddiv_rn((double)Ws, (double)Wr)), 0.5);
-      const double fy = floor(cy), fx = floor(cx);
-      const double ty = __dsub_rn(cy, fy), tx = __dsub_rn(cx, fx);
-      const int y0 = mirror_idx((int)fy, Hs), y1 = mirror_idx((int)fy + 1, Hs);
-      const int x0 = mirror_idx((int)fx, Ws), x1 = mirror_idx((int)fx + 1, Ws);
-      const double v00 = src[((size_t)y0 * Ws + x0) * 3 + ch], v01 = src[((size_t)y0 * Ws + x1) * 3 + ch];
-      const double v10 = src[((size_t)y1 * Ws + x0) * 3 + ch], v11 = src[((size_t)y1 * Ws + x1) * 3 + ch];
-      // scipy (ni_interpolation.c) sums the 2 x 2 neighbourhood, row-major, each term ((value * wy) * wx)
-      const double wy0 = __dsub_rn(1.0, ty), wx0 = __dsub_rn(1.0, tx);
-      double v = __dmul_rn(__dmul_rn(v00, wy0), wx0);
-      v = __dadd_rn(v, __dmul_rn(__dmul_rn(v01, wy0), tx));
-      v = __dadd_rn(v, __dmul_rn(__dmul_rn(v10, ty), wx0));
-      v = __dadd_rn(v, __dmul_rn(__dmul_rn(v11, ty), tx));
-      out = (unsigned char)fmin(fmax(trunc(v), 0.0), 255.0);
+#pragma unroll
+      for (int ch = 0; ch < 3; ++ch) px[ch] = zoom_px(fs, Hs, Ws, Hr, Wr, yr, xr, ch);
     }
-    dst[idx] = out;
+    float L, A, Bq;
+    rgb8_to_lab_px(px, &L, &A, &Bq);
+    l[idx] = L;
   }
 }
 
@@ -304,16 +330,16 @@ void launch_ctx_loss(const float* denom, float* loss, int B, int N, cudaStream_t
   ctx_loss_kernel<<<B, 256, 0, s>>>(denom, loss, N);
   launch_counter_add(1);
 }
-void launch_fgs_weights(const unsigned char* guide, const float* lut, float* Ch, float* Cv, int H, int W, cudaStream_t s) {
-  fgs_weights_kernel<<<grid_for((size_t)H * W, 256), 256, 0, s>>>(guide, lut, Ch, Cv, H, W);
+void launch_fgs_weights(const unsigned char* guide, const float* lut, float* Ch, float* Cv, int F, int H, int W, cudaStream_t s) {
+  fgs_weights_kernel<<<grid_for((size_t)F * H * W, 256), 256, 0, s>>>(guide, lut, Ch, Cv, F, H, W);
   launch_counter_add(1);
 }
-void launch_fgs_horizontal(float* cur, const float* Ch, float* D, int planes, int H, int W, float lam, cudaStream_t s) {
-  fgs_horizontal_kernel<<<planes * ((H + 31) / 32), 32, 0, s>>>(cur, Ch, D, planes, H, W, lam);
+void launch_fgs_horizontal(float* cur, const float* Ch, float* D, int planes, int ppg, int H, int W, float lam, cudaStream_t s) {
+  fgs_horizontal_kernel<<<planes * ((H + 31) / 32), 32, 0, s>>>(cur, Ch, D, planes, ppg, H, W, lam);
   launch_counter_add(1);
 }
-void launch_fgs_vertical(float* cur, const float* Cv, float* D, int planes, int H, int W, float lam, cudaStream_t s) {
-  fgs_vertical_kernel<<<(planes * W + 127) / 128, 128, 0, s>>>(cur, Cv, D, planes, H, W, lam);
+void launch_fgs_vertical(float* cur, const float* Cv, float* D, int planes, int ppg, int H, int W, float lam, cudaStream_t s) {
+  fgs_vertical_kernel<<<dim3((ppg * W + 127) / 128, planes / ppg), 128, 0, s>>>(cur, Cv, D, ppg, H, W, lam);
   launch_counter_add(1);
 }
 void launch_l_to_guide8(const float* l, unsigned char* g, size_t n, cudaStream_t s) {
@@ -333,6 +359,10 @@ void launch_gauss_axis_f64(const double* src, double* dst, const double* w, int 
 void launch_zoom_crop(const double* src, int Hs, int Ws, int Hr, int Wr, int oy, int ox, unsigned char* dst, int Ho, int Wo,
                       cudaStream_t s) {
   zoom_crop_kernel<<<grid_for((size_t)Ho * Wo * 3, 256), 256, 0, s>>>(src, Hs, Ws, Hr, Wr, oy, ox, dst, Ho, Wo);
+  launch_counter_add(1);
+}
+void launch_ingest_l(const double* src, int F, int Hs, int Ws, int Hr, int Wr, int oy, int ox, float* l, int Ho, int Wo, cudaStream_t s) {
+  ingest_l_kernel<<<grid_for((size_t)F * Ho * Wo, 256), 256, 0, s>>>(src, F, Hs, Ws, Hr, Wr, oy, ox, l, Ho, Wo);
   launch_counter_add(1);
 }
 

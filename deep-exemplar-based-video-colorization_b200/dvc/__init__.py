@@ -25,7 +25,7 @@ EXPORTED = [
     "dvc_resize_half", "dvc_upsample2_scaled", "dvc_lab_to_rgb8", "dvc_rgb8_to_lab",
     "dvc_fgs_filter", "dvc_l_to_guide8", "dvc_resize_antialias_crop_rgb8", "dvc_contextual_loss_forward",
     "dvc_peer_buffer_create", "dvc_peer_buffer_open", "dvc_peer_buffer_close", "dvc_peer_buffer_destroy",
-    "dvc_corr_set_peer_outputs",
+    "dvc_corr_set_peer_outputs", "dvc_ingest_rgb8", "dvc_postprocess_rgb8", "dvc_colorize_video_rgb8",
 ]
 
 _lib = None
@@ -84,6 +84,10 @@ def load_library():
         lib.dvc_l_to_guide8.argtypes = [c_void, c_void, c_int, c_int, c_void, c_void]
         lib.dvc_resize_antialias_crop_rgb8.argtypes = [c_void, c_void, c_int, c_int, c_int, c_int, c_int, c_int, c_void, c_int, c_int,
                                                        c_void]
+        lib.dvc_ingest_rgb8.argtypes = [c_void, c_void] + [c_int] * 9 + [c_void, c_void, c_void]
+        lib.dvc_postprocess_rgb8.argtypes = [c_void, c_void, c_void, c_int, c_int, c_int, c_int, c_float, c_float, c_void, c_void]
+        lib.dvc_colorize_video_rgb8.argtypes = ([c_void, c_void] + [c_int] * 9 + [c_float, c_int, c_float, c_float, c_int]
+                                                + [c_void, c_void])
         lib.dvc_contextual_loss_forward.argtypes = [c_void, c_void, c_void, c_int, c_int, c_int, c_int, c_float, c_int, c_void, c_void]
         lib.dvc_peer_buffer_create.argtypes = [c_void, c_i64, P(c_void), ctypes.c_char_p]
         lib.dvc_peer_buffer_open.argtypes = [c_void, ctypes.c_char_p, P(c_void)]
@@ -364,6 +368,70 @@ class Context:
         self._check(self.lib.dvc_resize_antialias_crop_rgb8(self.h, ctypes.c_void_p(rgb.data_ptr()), Hs, Ws, Hr, Wr, oy, ox,
                                                             ctypes.c_void_p(out.data_ptr()), size[0], size[1], _stream(rgb.device)),
                     "dvc_resize_antialias_crop_rgb8")
+        return out
+
+    # ---- whole frames in, whole frames out -------------------------------------------------------------
+    @staticmethod
+    def _geometry(Hs, Ws, size):
+        from dvc.prepost import centerpad_geometry
+
+        Ho, Wo = int(size[0]), int(size[1])
+        if Ho % 2 or Wo % 2:
+            raise DvcError("the output size must be even (the networks run at half of it)")
+        return centerpad_geometry(Hs, Ws, (Ho, Wo)) + (Ho, Wo)
+
+    def ingest_rgb8(self, frames, size):
+        """test.py:44-46,71 for CUDA uint8 frames [F,Hs,Ws,3]: CenterPad + CenterCrop to `size`, Lab, centred L only ->
+        (L [F,1,Ho,Wo], L at half size [F,1,Ho/2,Wo/2]).  Equals centerpad_rgb8 -> rgb8_to_lab -> [:, 0:1] -> resize_half."""
+        if not (isinstance(frames, torch.Tensor) and frames.is_cuda and frames.dtype == torch.uint8 and frames.dim() == 4
+                and frames.shape[3] == 3):
+            raise DvcError("ingest_rgb8: expected a CUDA uint8 tensor [F,H,W,3]")
+        frames = frames.contiguous()
+        F_, Hs, Ws, _ = frames.shape
+        Hr, Wr, oy, ox, Ho, Wo = self._geometry(Hs, Ws, size)
+        l = torch.empty(F_, 1, Ho, Wo, device=frames.device, dtype=torch.float32)
+        lh = torch.empty(F_, 1, Ho // 2, Wo // 2, device=frames.device, dtype=torch.float32)
+        self._check(self.lib.dvc_ingest_rgb8(self.h, ctypes.c_void_p(frames.data_ptr()), F_, Hs, Ws, Hr, Wr, oy, ox, Ho, Wo, _ptr(l),
+                                             _ptr(lh), _stream(frames.device)), "dvc_ingest_rgb8")
+        return l, lh
+
+    def postprocess_rgb8(self, l, ab_half, wls=True, lam=500.0, sigma_color=4.0):
+        """test.py:99-119 for CUDA l [F,1,Ho,Wo] (centred) and ab_half [F,2,Ho/2,Wo/2]: x2 * 1.25, the WLS filter guided by
+        each frame's own L (when wls), Lab -> sRGB uint8 [F,Ho,Wo,3]."""
+        l, ab_half = _dev_f32(l, "postprocess_rgb8 l"), _dev_f32(ab_half, "postprocess_rgb8 ab")
+        F_, c1, Ho, Wo = l.shape
+        if c1 != 1 or tuple(ab_half.shape) != (F_, 2, Ho // 2, Wo // 2):
+            raise DvcError("postprocess_rgb8: expected l [F,1,Ho,Wo] and ab [F,2,Ho/2,Wo/2]")
+        out = torch.empty(F_, Ho, Wo, 3, device=l.device, dtype=torch.uint8)
+        self._check(self.lib.dvc_postprocess_rgb8(self.h, _ptr(l), _ptr(ab_half), F_, Ho, Wo, 1 if wls else 0, float(lam),
+                                                  float(sigma_color), ctypes.c_void_p(out.data_ptr()), _stream(l.device)),
+                    "dvc_postprocess_rgb8")
+        return out
+
+    def colorize_video_rgb8(self, frames, size, temperature=1e-10, wls=True, lam=500.0, sigma_color=4.0, continue_clip=False,
+                            out=None):
+        """K frames of a clip, uint8 sRGB [K,Hs,Ws,3] -> colourised uint8 sRGB [K,size[0],size[1],3] (test.py:29-125 without
+        the file I/O), against the exemplar of set_exemplar, which must be size / 2.  continue_clip=True continues the
+        recurrence from the last frame of the previous call.  `frames` may be a (preferably pinned) CPU tensor or a CUDA
+        tensor; `out` lives where `frames` lives."""
+        if not (isinstance(frames, torch.Tensor) and frames.dtype == torch.uint8 and frames.dim() == 4 and frames.shape[3] == 3):
+            raise DvcError("colorize_video_rgb8 takes a uint8 tensor [K,H,W,3]")
+        if frames.shape[0] < 1:
+            raise DvcError("colorize_video_rgb8: no frames")
+        frames = frames.contiguous()
+        K, Hs, Ws, _ = frames.shape
+        Hr, Wr, oy, ox, Ho, Wo = self._geometry(Hs, Ws, size)
+        if out is None:
+            out = torch.empty(K, Ho, Wo, 3, dtype=torch.uint8, device=frames.device)
+            if not frames.is_cuda:
+                out = out.pin_memory()
+        if (out.is_cuda != frames.is_cuda or out.dtype != torch.uint8 or not out.is_contiguous()
+                or tuple(out.shape) != (K, Ho, Wo, 3)):
+            raise DvcError("colorize_video_rgb8: `out` must be a contiguous uint8 [K,Ho,Wo,3] tensor on the same side as the frames")
+        rc = self.lib.dvc_colorize_video_rgb8(self.h, ctypes.c_void_p(frames.data_ptr()), K, Hs, Ws, Hr, Wr, oy, ox, Ho, Wo,
+                                              float(temperature), 1 if wls else 0, float(lam), float(sigma_color),
+                                              1 if continue_clip else 0, ctypes.c_void_p(out.data_ptr()), _stream(self.device))
+        self._check(rc, "dvc_colorize_video_rgb8")
         return out
 
     # ---- query-row-sharded correlation: peer-mapped result buffers (CUDA IPC) ----------------------------

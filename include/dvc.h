@@ -172,6 +172,32 @@ int dvc_l_to_guide8(dvc_ctx* ctx, const float* dev_l, int H, int W, unsigned cha
 int dvc_resize_antialias_crop_rgb8(dvc_ctx* ctx, const unsigned char* dev_src, int Hs, int Ws, int Hr, int Wr, int oy, int ox,
                                    unsigned char* dev_dst, int Ho, int Wo, void* stream);
 
+/* ---- whole frames in, whole frames out ------------------------------------------------------------- */
+
+/* Frame ingest of test.py:44-46,71 for F frames dev_src [F,Hs,Ws,3] (uint8 sRGB, same size): CenterPad resize + crop / pad
+ * to [Ho,Wo] (geometry as for dvc_resize_antialias_crop_rgb8), sRGB -> Lab, and only the centred L is kept:
+ * dev_l [F,1,Ho,Wo] at full size and dev_l_half [F,1,Ho/2,Wo/2] (dvc_resize_half of it).  Bit for bit the chain
+ * dvc_resize_antialias_crop_rgb8 -> dvc_rgb8_to_lab -> channel 0 -> dvc_resize_half.  Ho and Wo must be even. */
+int dvc_ingest_rgb8(dvc_ctx* ctx, const unsigned char* dev_src, int F, int Hs, int Ws, int Hr, int Wr, int oy, int ox, int Ho,
+                    int Wo, float* dev_l, float* dev_l_half, void* stream);
+/* Output side of test.py:99-119 for F frames: ab at half size dev_ab_half [F,2,Ho/2,Wo/2] -> x2 * 1.25 -> (wls != 0) the
+ * Fast Global Smoother of each frame's two planes guided by its own luminance dev_l [F,1,Ho,Wo] (lambda, sigma_color,
+ * attenuation 0.25, 3 iterations) -> sRGB uint8 dev_rgb [F,Ho,Wo,3].  Bit for bit dvc_upsample2_scaled(1.25) -> per frame
+ * dvc_l_to_guide8 + dvc_fgs_filter -> dvc_lab_to_rgb8, in one launch per step for all F frames. */
+int dvc_postprocess_rgb8(dvc_ctx* ctx, const float* dev_l, const float* dev_ab_half, int F, int Ho, int Wo, int wls, float lambda,
+                         float sigma_color, unsigned char* dev_rgb, void* stream);
+/* Colourise K consecutive frames of a clip, uint8 sRGB in and out: host_src [K,Hs,Ws,3] -> dvc_ingest_rgb8 -> the networks
+ * with the recurrence of test.py:76-96 (as dvc_colorize_clip) -> dvc_postprocess_rgb8 -> host_dst [K,Ho,Wo,3].  The nets
+ * run at Ho/2 x Wo/2, which must be the size of the exemplar given to dvc_set_exemplar.  continue_clip = 0 starts the
+ * recurrence from zeros (test.py:80); continue_clip = 1 continues it from the last frame of the previous call, which
+ * must have succeeded against the same exemplar and the same Ho x Wo (otherwise DVC_ERR_STATE) -- the source size may
+ * change between calls.  A clip of any length can so be fed in chunks: device memory depends on the frame sizes only,
+ * never on K.  host_src / host_dst may be host (pinned for full overlap) or device memory.  Synchronises `stream`
+ * before returning. */
+int dvc_colorize_video_rgb8(dvc_ctx* ctx, const unsigned char* host_src, int K, int Hs, int Ws, int Hr, int Wr, int oy, int ox,
+                            int Ho, int Wo, float temperature, int wls, float lambda, float sigma_color, int continue_clip,
+                            unsigned char* host_dst, void* stream);
+
 /* ---- multi-GPU: exemplar operands travel once per clip (SURVEY.md §8e) ----------------------- */
 
 /* ---- single-frame scaling: query-row-sharded correlation with a fused all-gather (SURVEY.md §8e, BASELINE config 4) --

@@ -1,10 +1,11 @@
 """The reference's test.py:29-125 data flow on the device, using only libdvc entry points (no reference code):
 
-    decoded uint8 frames -> CenterPad + CenterCrop to --image_size (dvc_resize_antialias_crop_rgb8) -> Lab
-    (dvc_rgb8_to_lab) -> 1/2 resolution (dvc_resize_half) -> exemplar features once (dvc_set_exemplar) -> per frame
-    VGG19 / WarpNet / correlation / ColorVidNet with the recurrence kept on the device (dvc_colorize_clip) -> ab x2 * 1.25
-    (dvc_upsample2_scaled) -> WLS filter guided by the full-resolution luminance (dvc_l_to_guide8 + dvc_fgs_filter,
-    test.py:105-112) -> sRGB uint8 (dvc_lab_to_rgb8) -> PNG files
+    PNG files decoded on a thread pool -> chunks of uint8 frames (dvc/stream.py: colorize_stream) -> per chunk one
+    dvc_colorize_video_rgb8 call: CenterPad + CenterCrop to --image_size, Lab, 1/2 resolution (dvc_ingest_rgb8) -> per
+    frame VGG19 / WarpNet / correlation / ColorVidNet with the recurrence kept on the device (the dvc_colorize_clip
+    driver) -> ab x2 * 1.25 -> WLS filter guided by the full-resolution luminance (test.py:105-112) -> sRGB uint8
+    (dvc_postprocess_rgb8) -> PNG files.  The exemplar goes through dvc_resize_antialias_crop_rgb8 -> dvc_rgb8_to_lab ->
+    dvc_resize_half -> dvc_set_exemplar once.  Memory does not grow with the length of the clip.
 
     python tools/colorize_folder.py --clip frames/ --ref exemplar.png --out out/ \
         --vgg vgg19_conv.pth --warp nonlocal_net_iter_76000.pth --color colornet_iter_76000.pth
@@ -42,6 +43,7 @@ def main():
     ap.add_argument("--no-wls", action="store_true", help="skip the Fast Global Smoother (test.py:31 wls_filter_on)")
     ap.add_argument("--lambda-value", type=float, default=500.0)  # test.py:32
     ap.add_argument("--sigma-color", type=float, default=4.0)    # test.py:33
+    ap.add_argument("--workers", type=int, default=min(8, os.cpu_count() or 1), help="PNG decode threads")
     args = ap.parse_args()
 
     import dvc
@@ -60,28 +62,17 @@ def main():
     H, W = args.image_size
     if H % 16 or W % 32:
         raise SystemExit("--image-size must have H % 16 == 0 and W % 32 == 0 (the networks run at half of it)")
-    # test.py:44-46: CenterPad(image_size) + CenterCrop(image_size), anti-aliased resize on the device
-    frames = torch.stack([ctx.centerpad_rgb8(load_rgb8(os.path.join(args.clip, n)).cuda(), (H, W)) for n in names])  # [F,H,W,3]
-    ref = ctx.centerpad_rgb8(load_rgb8(args.ref).cuda(), (H, W))[None]
-    F_ = frames.shape[0]
-
-    lab_large = ctx.rgb8_to_lab(frames)                      # [F,3,H,W], centred L   (test.py:44-45)
-    lab = ctx.resize_half(lab_large)                         # test.py:71
-    ctx.set_exemplar(ctx.resize_half(ctx.rgb8_to_lab(ref)))  # test.py:57-66
-    ab = ctx.colorize_clip(lab[:, 0:1].contiguous(), args.temperature)  # test.py:68-96, recurrence on the device
-    ab_large = ctx.upsample2_scaled(ab, 1.25)                # test.py:100-102
-    if not args.no_wls:                                      # test.py:105-112
-        for t in range(F_):
-            guide = ctx.l_to_guide8(lab_large[t, 0])
-            ab_large[t] = ctx.fgs_filter(guide, ab_large[t], args.lambda_value, args.sigma_color)
-    rgb = ctx.lab_to_rgb8(lab_large[:, 0:1].contiguous(), ab_large).cpu().numpy()  # test.py:116-119
-
     from PIL import Image
 
+    from dvc.stream import colorize_stream
+
     os.makedirs(args.out, exist_ok=True)
-    for n, img in zip(names, rgb):
+    frames = colorize_stream(ctx, (os.path.join(args.clip, n) for n in names), load_rgb8(args.ref), (H, W), args.temperature,
+                             wls=not args.no_wls, lam=args.lambda_value, sigma_color=args.sigma_color, decode=load_rgb8,
+                             workers=args.workers)
+    for n, img in zip(names, frames):
         Image.fromarray(img).save(os.path.join(args.out, os.path.splitext(n)[0] + ".png"))
-    print(f"{F_} frames -> {args.out}")
+    print(f"{len(names)} frames -> {args.out}")
 
 
 if __name__ == "__main__":
