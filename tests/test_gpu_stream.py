@@ -40,7 +40,9 @@ def chain_post(ctx, l, ab, wls, lam=500.0, sigma=4.0):
 
 
 def composition(ctx, frames, ref, size, wls=True):
-    """tools/colorize_folder.py's data flow before it streamed: every frame decoded up front, every step over the clip."""
+    """tools/colorize_folder.py's data flow before it streamed: every frame decoded up front, every step over the clip.
+    `frames` is a uint8 [F,H,W,3] tensor or a list of uint8 [H,W,3] frames whose sizes may differ (each is CenterPad-ed
+    to `size` on its own)."""
     big = torch.stack([ctx.centerpad_rgb8(f.cuda(), size) for f in frames])
     lab_large = ctx.rgb8_to_lab(big)
     lab = ctx.resize_half(lab_large)
@@ -85,13 +87,78 @@ def clip11():
     return frames, ref
 
 
+@pytest.fixture
+def flags(ctx):
+    """ctx.debug_flag for one test; the shipped values come back afterwards, also when the test fails."""
+    yield ctx.debug_flag
+    ctx.debug_flag("video_batch", 8)
+    ctx.debug_flag("clip_astreams", 1)
+
+
+def video_calls(ctx, frames, sizes, wls=True):
+    """The clip in consecutive calls of `sizes` frames, the recurrence continued across them."""
+    pinned, out, t = frames.pin_memory(), [], 0
+    for k in sizes:
+        out.append(ctx.colorize_video_rgb8(pinned[t:t + k], SIZE, wls=wls, continue_clip=t > 0))
+        t += k
+    assert t == len(frames)
+    return torch.cat(out)
+
+
 @pytest.mark.parametrize("wls", [True, False])
 @pytest.mark.parametrize("K", [1, 4, 11])
-def test_streamed_chunks_equal_composition(ctx, clip11, K, wls):
+@pytest.mark.parametrize("G", [1, 3, 8])
+def test_streamed_chunks_equal_composition(ctx, flags, clip11, G, K, wls):
+    """G frames per post-processing batch: batch b uses half b & 1 of the L and ab rings, so G = 1 and 3 wrap them several
+    times inside one call, G = 3 with K = 11 ends in a partial batch of 2 after a wrap, and K = 4 with G = 3 puts call
+    boundaries in the middle of a batch."""
     frames, ref = clip11
     want = composition(ctx, frames, ref, SIZE, wls)  # also installs the exemplar
-    pinned = frames.pin_memory()
-    got = torch.cat([ctx.colorize_video_rgb8(pinned[t:t + K], SIZE, wls=wls, continue_clip=t > 0) for t in range(0, 11, K)])
+    flags("video_batch", G)
+    got = video_calls(ctx, frames, [min(K, 11 - t) for t in range(0, 11, K)], wls)
+    assert torch.equal(got, want)
+
+
+@pytest.fixture(scope="module")
+def clip40():
+    return seeded_frames(41, 40, 90, 120), seeded_frames(42, 1, 90, 120)[0]
+
+
+@pytest.mark.parametrize("wls", [True, False])
+@pytest.mark.parametrize("sizes,astreams", [((40,), 1), ((17, 23), 1), ((37, 3), 1), ((17, 23), 2)])
+def test_video_rings_wrap_at_the_default_batch(ctx, flags, clip40, sizes, astreams, wls):
+    """The shipped G = 8 past 2G frames in one call, where ingest and ColorVidNet wait for batch b - 2's post-processing
+    before they reuse its ring slots: 40 frames are five batches (the rings wrap twice, the last batch is full); 17 + 23
+    and 37 + 3 put the call boundary in the middle of a batch.  clip_astreams = 2 has frames t+1 and t+2 in flight on two
+    phase-A streams."""
+    frames, ref = clip40
+    want = composition(ctx, frames, ref, SIZE, wls)
+    flags("clip_astreams", astreams)
+    assert torch.equal(video_calls(ctx, frames, sizes, wls), want)
+
+
+def test_source_size_changes_mid_clip(ctx, clip11):
+    """Runs of 90 x 120, 150 x 180, 90 x 120 and 100 x 300 frames, each longer than 2G: the source frame and the ingest work
+    buffers regrow in the middle of a continued clip.  Once with one call per run, once through colorize_stream, which
+    ends a chunk at each size change."""
+    _, ref = clip11
+    runs = [seeded_frames(50 + i, n, h, w) for i, (n, h, w) in enumerate([(18, 90, 120), (22, 150, 180), (19, 90, 120), (18, 100, 300)])]
+    frames = [f for run in runs for f in run]
+    want = composition(ctx, frames, ref, SIZE)
+    got = torch.cat([ctx.colorize_video_rgb8(run.pin_memory(), SIZE, continue_clip=i > 0) for i, run in enumerate(runs)])
+    assert torch.equal(got, want)
+    streamed = list(colorize_stream(ctx, iter([f.numpy() for f in frames]), ref.numpy(), SIZE, chunk=20, workers=2))
+    assert torch.equal(torch.from_numpy(np.stack(streamed)), want)
+
+
+def test_product_geometry(ctx):
+    """The geometry of profiles/stream_bench.json: 1080 x 1920 sources at image_size 960 x 1728 (the nets at 480 x 864), 20
+    frames in one call with the WLS filter: rings at full size, FGS batched over 8 frames of 960 x 1728."""
+    frames = torch.cat([seeded_frames(61 + t, 1, 1080, 1920) for t in range(20)])  # 124 MB; one frame of noise at a time
+    ref = seeded_frames(62, 1, 1080, 1920)[0]
+    size = (960, 1728)
+    want = composition(ctx, frames, ref, size)
+    got = ctx.colorize_video_rgb8(frames.pin_memory(), size, continue_clip=False)
     assert torch.equal(got, want)
 
 
